@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — reprojection residuals/sec and LM iterations/sec of the bundle-adjustment hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one full `bundle_adjust()` (calibration.py:199-212 semantics: ftol=1e-4, max_nfev=100, linear loss) over one
 synthetic scene of the BASELINE.json configuration `--workload`.  Default workload at EVERY N: cfg4 = configs[3] (16 cameras x
@@ -15,6 +15,10 @@ Metric (both arms, same definition):
 `value`  : solves timed on the device with the packed problem already resident in HBM (CUDA events on the solver's stream).
 `e2e`    : the same through the public API `Calibration.bundle_adjust()` from pinned host numpy buffers: packing, H2D, solve, D2H of
            the solved parameters all inside the timed region (wall clock, device synchronised).
+Each workload block times exactly `--steps` solves per path (the reference arm below may stop earlier, at `--ref-budget-s`).
+`--dump-outputs DIR` writes what the last timed device-resident solve of `--workload` returned, as DIR/<name>.npy (float64): the solved
+parameter vector, the solve summary and iteration log, and the residuals at the solution (a fixed, seeded sample of them).  The inputs
+depend only on the arguments, so two builds run with the same arguments can be compared output for output.
 `--impl reference` times the reference's CPU path on the host cores on a bounded frame-subsample of the same workload: the
 unmodified reference (through tests/refshim) where /root/reference exists (the build container), else its numpy + scipy restatement
 oracle/ba_oracle.py (the GPU box: the reference is pure Python and cannot travel); `cpu_baseline.kind` says which.
@@ -35,6 +39,28 @@ sys.path.insert(0, ROOT)
 METRIC, UNIT = "reprojection_residuals_per_sec", "residuals/s"
 BA_KW = dict(tolerance=1e-4, max_iterations=100, loss="linear", f_scale=1.0)
 REF_FRAMES = {"cfg1": 20, "cfg2": 20, "cfg3": 12, "cfg4": 8, "cfg5": 2}      # CPU sample: ~10-40 s of scipy TRF + finite differences
+DUMP_RESIDUALS = 1 << 20                  # residuals written by --dump-outputs: 8 MiB, plus their indices
+
+
+def dump_outputs(directory, eng, res):
+  """The arrays the last timed solve handed its caller: solved parameters (reference order), [cost, initial_cost, optimality, nfev,
+  njev, status], the iteration log as (iteration, nfev, cost, optimality) per row and (cost_reduction, step_norm) per step taken (row 0
+  is the starting point: no step, logged as NaN, so it is left out), and the residuals at the solution, all of them or DUMP_RESIDUALS
+  of them at fixed, seeded positions (residuals_index).  Every array written is finite."""
+  os.makedirs(directory, exist_ok=True)
+  r = eng.residuals()
+  idx = np.arange(r.size)
+  if r.size > DUMP_RESIDUALS:
+    idx = np.sort(np.random.default_rng(0).choice(r.size, DUMP_RESIDUALS, replace=False))
+  log = np.array(res.log, dtype=np.float64).reshape(-1, 6)
+  arrays = dict(param_vec=eng.param_vec,
+                solve_summary=np.array([res.cost, res.initial_cost, res.optimality, res.nfev, res.njev, res.status], dtype=np.float64),
+                iteration_log=log[:, [0, 1, 2, 5]], step_log=log[1:, 3:5],
+                residuals=r[idx], residuals_index=idx.astype(np.float64))
+  for name, a in arrays.items():
+    if not np.isfinite(a).all(): raise RuntimeError(f"--dump-outputs: {name} of the last solve is not finite")
+  for name, a in arrays.items():
+    np.save(os.path.join(directory, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def subsample_frames(scene, frames):
@@ -238,8 +264,9 @@ def run_ours(args):
   if world > 1:
     mdist.init_comm(eng, rank, world)
 
-  def measure(local_scene, steps, warmup, e2e=True, roofline=True):
-    """Device-resident solves, end-to-end solves and the linearisation kernel's roofline point for one (sharded) scene."""
+  def measure(local_scene, steps, warmup, e2e=True, roofline=True, dump_dir=None):
+    """Device-resident solves, end-to-end solves and the linearisation kernel's roofline point for one (sharded) scene; with
+    `dump_dir`, rank 0 writes the outputs of the last resident solve there."""
     calib = from_scene(local_scene).enable(cameras=True)
     n_total = allsum_int(int(calib.inliers.sum()))
     state0 = calib._state_arrays()
@@ -260,6 +287,7 @@ def run_ours(args):
       res, ms = solve_resident()
       t_dev += ms; evals += res.nfev + res.njev; njev += res.njev; launches += res.kernel_launches; last = res
     barrier()
+    if dump_dir and rank == 0: dump_outputs(dump_dir, eng, last)          # before the e2e solves below reuse the engine
     t_dev = allmax(t_dev)
     out = dict(corners=n_total, ms_per_step=t_dev / steps, value=n_total * evals / (t_dev * 1e-3), lm_iters_per_sec=njev / (t_dev * 1e-3),
                nfev_plus_njev_per_step=evals / steps, gpu_launches=launches, cost=last.cost, nfev=last.nfev, params=eng.num_params)
@@ -304,7 +332,7 @@ def run_ours(args):
   scene = synthetic.make_workload(args.workload, seed=args.seed)
   my = mdist.frame_range(scene["F"], rank, world)
   local_scene = pin(subsample_frames(scene, np.arange(*my)) if world > 1 else scene)
-  main, calib = measure(local_scene, args.steps, args.warmup)
+  main, calib = measure(local_scene, args.steps, args.warmup, dump_dir=args.dump_outputs)
 
   # the same end-to-end call over a float32 table: make_point_table keeps the dtype of the detector's corners (tables.py:15-17; cv2 returns
   # float32), so for real detections THIS is the reference's table.  The scene is the main scene rounded to float32 (8 B per entry over the link).
@@ -336,7 +364,7 @@ def run_ours(args):
   if world == 1 and args.secondary:
     for wl in ("cfg2", "cfg3", "cfg5"):      # cfg5 = BASELINE configs[4] (64 cameras x 2000 frames, 50.8 M corners, n_s = 1030): it fits one GPU as well
       if wl == args.workload: continue
-      o, _ = measure(pin(synthetic.make_workload(wl, seed=args.seed)), max(3, args.steps // 2), args.warmup)
+      o, _ = measure(pin(synthetic.make_workload(wl, seed=args.seed)), args.steps, args.warmup)
       o.pop("cost", None)
       others[wl] = o
   if world > 1:
@@ -360,7 +388,7 @@ def run_ours(args):
       base = dict(synthetic.WORKLOADS["cfg2"])
       wscene = synthetic.make_scene(seed=args.seed, **{**base, "F": base["F"] * world})
       wmy = mdist.frame_range(wscene["F"], rank, world)
-      o, _ = measure(pin(subsample_frames(wscene, np.arange(*wmy))), max(3, args.steps // 2), args.warmup, e2e=False, roofline=False)
+      o, _ = measure(pin(subsample_frames(wscene, np.arange(*wmy))), args.steps, args.warmup, e2e=False, roofline=False)
       o.pop("cost", None)
       others["weak_cfg2_per_gpu"] = dict(o, scaling="weak", frames_per_gpu=base["F"])
   sampler.stop_flag = True; sampler.join(timeout=2)
@@ -421,12 +449,14 @@ def main():
   ap.add_argument("--ref-frames", type=int, default=0, help="frames in the CPU-baseline sample (0: per-workload default)")
   ap.add_argument("--ref-budget-s", type=float, default=240.0, help="the reference arm stops taking steps after this many seconds")
   ap.add_argument("--no-secondary", dest="secondary", action="store_false", help="skip the secondary workload blocks")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write the outputs of the last timed solve to DIR/<name>.npy")
   args = ap.parse_args()
+  if args.steps < 1: ap.error("--steps must be at least 1")
   if args.impl == "reference":
     run_reference(args)
   else:
     import __graft_entry__ as g
-    g.build()
+    if os.access(os.path.dirname(g.LIB), os.W_OK): g.build()     # a read-only tree runs the library build() left there as it is
     run_ours(args)
 
 

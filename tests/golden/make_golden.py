@@ -175,9 +175,69 @@ def pnp_cases(ref, only):
     print(name, "views", table.valid.size, "valid", int(table.valid.sum()), "max err", float(np.max(table.reprojection_error)), os.path.getsize(path) // 1024, "KB")
 
 
+def scene_arrays(scene, src):
+  """The inputs of a scene in the layout tests/conftest.py load_golden reads (src: the scene's "init" or "gt" estimates)."""
+  return dict(model=scene["model"], points=scene["points"], valid=scene["valid"],
+              cam_valid=scene["cam_valid"], frame_valid=scene["frame_valid"], board_valid=scene["board_valid"],
+              board_points=np.stack(scene["board_points"]), K=src["K"], dist=src["dist"],
+              cam_poses=src["cam_poses"], frame_poses=src["frame_poses"], board_poses=src["board_poses"],
+              image_size=np.array(scene["image_size"]))
+
+
+def dome_case(ref, name="dome_cube2_3x5"):
+  """Three cameras on a dome around two 10x10 cube faces (tests/test_oracle.py test_oracle_against_reference_dome_rig):
+    x0            Calibration.param_vec
+    x1, r1        a perturbed parameter vector and the reference's residuals there
+    sp_*          Calibration.sparsity_matrix (CSR, sorted indices, with its values)"""
+  scene = synthetic.make_scene(C=3, F=5, vis=0.6, seed=21, boards=("cube", 10, 10, 0.04, 2), rig="dome")
+  calib = loader.build_calibration(ref, scene).enable(cameras=True)
+  x0 = calib.param_vec
+  x1 = x0 + np.random.default_rng(5).normal(0, 1e-3, x0.size)
+  c1 = calib.with_param_vec(x1)
+  r1 = (c1.reprojected.points - c1.point_table.points)[calib.inliers].ravel()
+  S = calib.sparsity_matrix.tocsr(); S.sort_indices()
+  data = dict(scene_arrays(scene, scene["init"]), cameras_enabled=True, x0=x0, x1=x1, r1=r1,
+              sp_indptr=S.indptr, sp_indices=S.indices, sp_data=S.data, sp_shape=np.array(S.shape))
+  path = os.path.join(HERE, name + ".npz")
+  np.savez_compressed(path, **data)
+  print(name, "N", int(calib.inliers.sum()), "n", x0.size, os.path.getsize(path) // 1024, "KB")
+
+
+def reference_calibration_cases(ref, only):
+  """What tests/test_simt_kernels.py test_calibration_over_the_reference_objects compares this package's Calibration against, for
+  the static, rolling and hand-eye motion models of one small scene (the motion inputs are stored beside the scene):
+    x0                   Calibration.param_vec
+    ok, reprojected      reprojected.valid & point_table.valid, and reprojected.points where it holds
+    reprojection_error   Calibration.reprojection_error
+    cost0                half the squared inlier residuals at x0"""
+  for motion in ("static", "rolling", "hand_eye"):
+    name = "refcalib_" + motion
+    if only and name not in only: continue
+    scene = synthetic.make_scene(C=2, F=5, vis=0.4, seed=77)
+    spec, extra = None, {}
+    if motion == "rolling":
+      end = scene["init"]["frame_poses"].copy(); end[:, :3, 3] += 0.005
+      spec, extra = ("rolling", end), dict(frame_poses_end=end)
+    elif motion == "hand_eye":
+      spec = ("hand_eye", scene["init"]["frame_poses"], np.eye(4), np.eye(4))          # arm poses = frame estimates, identity hand-eye pair
+      extra = dict(base_wrt_gripper=spec[1], world_wrt_base=spec[2], gripper_wrt_camera=spec[3])
+    rc = loader.build_calibration(ref, scene, motion=spec)
+    rc = rc.enable(camera_poses=False, cameras=False) if motion == "hand_eye" else rc.enable(cameras=True)
+    ok = np.asarray(rc.reprojected.valid) & np.asarray(rc.point_table.valid)
+    r0 = (np.asarray(rc.reprojected.points) - np.asarray(rc.point_table.points))[np.asarray(rc.inliers)]
+    data = dict(scene_arrays(scene, scene["init"]), motion=motion, x0=np.asarray(rc.param_vec), ok=ok,
+                reprojected=np.asarray(rc.reprojected.points)[ok], reprojection_error=np.asarray(rc.reprojection_error),
+                cost0=0.5 * float(np.sum(r0 ** 2)), **extra)
+    path = os.path.join(HERE, name + ".npz")
+    np.savez_compressed(path, **data)
+    print(name, "n", data["x0"].size, "ok", int(ok.sum()), "cost0", data["cost0"], os.path.getsize(path) // 1024, "KB")
+
+
 def main():
   ref = loader.load()
   only = sys.argv[1:]          # optional: regenerate just the named cases (existing fixtures stay byte-identical)
+  if not only or "dome_cube2_3x5" in only: dome_case(ref)
+  if not only or any(n.startswith("refcalib_") for n in only): reference_calibration_cases(ref, only)
   if not only or "outliers_3x6" in only: outlier_case(ref)
   if not only or any(n in only for n in ("rolling_2x6", "handeye_2x6")): motion_cases(ref, only)
   if not only or any(n.startswith("pnp_") for n in only): pnp_cases(ref, only)

@@ -209,6 +209,34 @@ def test_calibration_over_the_reference_objects(motion):
   assert out.last_solve.cost < 0.5 * float(np.sum(((np.asarray(rc.reprojected.points) - np.asarray(rc.point_table.points))[np.asarray(rc.inliers)]) ** 2))
 
 
+@pytest.mark.parametrize("motion", ["static", "rolling", "hand_eye"])
+def test_calibration_matches_the_reference_calibration_golden(motion):
+  """The comparisons of test_calibration_over_the_reference_objects against what the reference's own Calibration computed on the same
+  scene (tests/golden/make_golden.py reference_calibration_cases), with this package's mirror objects in place of the reference's:
+  parameter vector, projections and reprojection errors equal the reference's, and bundle_adjust keeps the object classes and lowers
+  the reference's initial cost."""
+  import numpy as np
+  from conftest import load_golden
+  from multical_b200.calibration import from_scene
+  from multical_b200.motion import HandEye, RollingFrames
+  from multical_b200.pose_set import pose_table
+  scene, z = load_golden("refcalib_" + motion)
+  calib = from_scene(scene)
+  if motion == "rolling":
+    calib = calib.copy(motion=RollingFrames(z["frame_poses"], z["frame_poses_end"], z["frame_valid"], [str(i) for i in range(scene["F"])]))
+  elif motion == "hand_eye":
+    calib = calib.copy(motion=HandEye(pose_table(z["base_wrt_gripper"], z["frame_valid"]), z["world_wrt_base"], z["gripper_wrt_camera"]))
+  calib = calib.enable(camera_poses=False, cameras=False) if motion == "hand_eye" else calib.enable(cameras=True)
+  assert np.abs(np.asarray(calib.param_vec) - z["x0"]).max() < 1e-12
+  assert np.abs(np.asarray(calib.reprojected.points)[z["ok"]] - z["reprojected"]).max() < 1e-9
+  assert np.abs(np.asarray(calib.reprojection_error) - z["reprojection_error"]).max() < 1e-9
+  out = calib.bundle_adjust(max_iterations=10)
+  assert type(out.motion) is type(calib.motion) and type(out.cameras[0]) is type(calib.cameras[0])
+  r = (np.asarray(out.reprojected.points) - np.asarray(out.point_table.points))[np.asarray(out.inliers)]
+  assert abs(0.5 * float(np.sum(r ** 2)) - out.last_solve.cost) <= 1e-9 * out.last_solve.cost
+  assert out.last_solve.cost < float(z["cost0"])
+
+
 def test_cfg1_the_reference_cpu_case_end_to_end():
   """BASELINE.json configs[0] (2 cameras x 20 frames of charuco_16x22, ~5k corners: the case the reference itself runs on the CPU):
   Calibration.bundle_adjust through the C-ABI against the reference algorithm (oracle: dense numpy evaluate + the identical scipy call)."""
