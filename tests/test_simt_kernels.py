@@ -16,6 +16,7 @@ import test_gpu_parity as gp
 import test_gpu_table as gt
 import test_gpu_motion as gm
 import test_gpu_pnp as gn
+import test_lm_step as ls
 from multical_b200 import _native, calibration
 
 
@@ -145,6 +146,29 @@ test_pnp_pose_table_matches_reference_golden = gn.test_pose_table_matches_refere
 test_pnp_every_camera_model_against_opencv = gn.test_every_camera_model_against_opencv
 test_pnp_minimum_detections_rule_and_bad_inputs = gn.test_minimum_detections_rule_and_bad_inputs
 test_pnp_april_grid_style_ids_use_the_tag_grid = gn.test_april_grid_style_ids_use_the_tag_grid
+
+
+# ---- tests/test_lm_step.py on the interpreter (one k_lm step against the refined dense model; n_s = 129 and 161 at three grid sizes below)
+_GRID_CASES = ("ns129_full", "ns161_rolling")
+
+
+@pytest.mark.parametrize("name", [c for c in ls.CASES if c not in _GRID_CASES and (c != "ns1030_full" or os.environ.get("MCBA_SIMT_FULL") == "1")])
+def test_lm_first_step_matches_the_refined_dense_model(name):
+  ls.check_first_step(name)
+
+
+@pytest.mark.parametrize("sms", [1, 3, None])
+@pytest.mark.parametrize("name", _GRID_CASES)
+def test_lm_first_step_at_three_grid_sizes(name, sms, monkeypatch):
+  """SIMT_SMS (the SM count the interpreter reports, read when the context is created): 1 -> k_lm on one CTA, where one CTA also works
+  off every trailing-update tile of the blocked factorisation; 3 -> CTA 0 plus two helpers; default (148, a B200) -> the launch shape of
+  the GPU suite."""
+  if sms is not None: monkeypatch.setenv("SIMT_SMS", str(sms))
+  ls.check_first_step(name)
+
+
+test_lm_rejected_trial_then_boundary_step_on_the_blocked_path = ls.test_rejected_trial_then_boundary_step_on_the_blocked_path
+test_lm_iteration_table_matches_the_model_on_device_normal_equations = ls.test_iteration_table_matches_the_model_on_device_normal_equations
 
 
 def test_the_product_refuses_the_interpreter_build(simt_library, monkeypatch):
